@@ -1,12 +1,15 @@
 #!/usr/bin/env python
 """bench.py — attention-forward throughput of the B200 path on BASELINE.json's headline configuration.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N --steps K --warmup W      (N > 1)
 
 A "step" is one forward of the drop-in ``ViT.Attention(768, 12)`` over one batch of synthetic tokens
 (BASELINE.json configs[1]: B=64 per GPU, N=197, d=768, heads=12; weak scaling: each rank has its own batch,
 no collective on the data path).  Rank 0 prints ONE JSON line; see DESIGN.md §Measurement for every field.
+
+--dump-outputs DIR: after the timed steps, rank 0 writes the output of the last timed step, y [B, N, C], as DIR/y.npy
+(float32).  Inputs and parameters are seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -269,8 +272,8 @@ def run_ours(args, rank, world, local):
         def step(i):
             if graphs:
                 graphs[i % RING].replay()
-            else:
-                outs_local = mod(xs[i % RING])   # noqa: F841
+                return outs[i % RING]
+            return mod(xs[i % RING])
 
         for i in range(max(args.warmup, 3)):
             step(i)
@@ -283,11 +286,15 @@ def run_ours(args, rank, world, local):
         torch.cuda.synchronize()
         e0.record()
         for i in range(args.steps):
-            step(i)
+            y_last = step(i)
         e1.record()
         torch.cuda.synchronize()
         sampler.stop_flag = True
         sampler.join()
+        if args.dump_outputs and rank == 0:
+            import numpy as np
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            np.save(os.path.join(args.dump_outputs, "y.npy"), y_last.float().cpu().numpy())
         barrier(world)
         launches = (_lib.launch_count() - l0) if not graphs else launches_per_forward * args.steps
         elapsed_ms = max_over_ranks(e0.elapsed_time(e1), world, dev)
@@ -453,7 +460,12 @@ def main():
     ap.add_argument("--no-fused", action="store_true", help="three launches (qkv GEMM, attention, proj GEMM) instead of a single-launch kernel")
     ap.add_argument("--no-other-configs", action="store_true", help="skip the side measurements of the other BASELINE configurations")
     ap.add_argument("--no-cosched", action="store_true", help="sequenced single-launch kernel instead of the co-scheduled one")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's output to DIR/y.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the output of the B200 path (--impl ours)")
     if args.no_fused:
         os.environ["PA_VIT_FUSED"] = "0"
     if args.no_cosched:

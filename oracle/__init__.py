@@ -13,8 +13,9 @@ reference itself: ``oracle/make_golden.py`` imports the real modules from
 restatement against them (fp32, <= 2e-6 max-abs) and commits seeded
 input/output vectors under ``tests/golden/``.  ``tests/test_oracle_golden.py``
 re-checks the restatement against those committed vectors on every run, and
-``tests/test_oracle_vs_reference.py`` re-checks against the live reference
-whenever ``/root/reference`` is mounted.
+``tests/test_oracle_vs_reference.py`` re-checks against further reference
+outputs (fresh seeds, configurations without a golden file) that
+``oracle/record_reference.py`` recorded into ``tests/golden/reference/fresh_seeds.npz``.
 """
 from .attention import (  # noqa: F401
     vit_attention,

@@ -6,8 +6,10 @@ A *spec* is a plain dict: {"variant", "ctor": {...}, "x": shape tuple, extra}.
 from __future__ import annotations
 
 import importlib
+import math
 import sys
 
+import numpy as np
 import torch
 
 from . import attention as A
@@ -66,6 +68,20 @@ GOLDEN_CASES = {
     "xcablock_b2_n196_c128_h2": dict(variant="xca_block", ctor=dict(dim=128, num_heads=2, qkv_bias=True, eta=1.0), x=(2, 196, 128),
                                      keep=("norm1.", "attn.", "gamma1")),
 }
+
+EXTRA_SPECS = {
+    # configurations of the GPU oracle cases that have no golden file of their own: tests/golden/reference/fresh_seeds.npz holds the
+    # reference's outputs for them, so those GPU cases are pinned through it
+    "xca_nano_hd32": dict(variant="xca", ctor=dict(dim=128, num_heads=4), x=(3, 196, 128)),
+    "classattn_nano_hd32": dict(variant="class_attn", ctor=dict(dim=128, num_heads=4), x=(3, 197, 128)),
+    "vit_l_like": dict(variant="vit", ctor=dict(dim=256, num_heads=4), x=(2, 197, 256)),
+}
+
+# bvit.Broad_Attention configurations whose four outputs (out, q, k, v) are recorded: inner width != dim, and heads == 1 with
+# dim_head == dim, where there is no output projection (bvit.py:52, 61-64)
+BVIT_QKV_CTORS = [dict(dim=192, heads=3, dim_head=64), dict(dim=64, heads=1, dim_head=64)]
+
+SAMPLE = 512        # elements of each recorded reference output kept in tests/golden/reference/fresh_seeds.npz
 
 _REF_CLASS = {
     "vit": ("ViT", "Attention"),
@@ -145,6 +161,46 @@ def make_inputs(spec, seed=0):
         out["dconv_weight"] = round_fp16_(torch.randn(L_, c["dim"], 1, 3, 3, generator=g) / 3.0)
         out["dconv_bias"] = round_fp16_(torch.randn(L_, c["dim"], generator=g) * 0.05)
     return out
+
+
+def shuffled_case(inputs, params, seed):
+    """A fresh case drawn from a stored one: the elements of every floating tensor permuted by a seeded generator.  Each
+    tensor keeps its values (BN variances stay positive, LayerNorm weights near one, all fp16-representable) at new places."""
+    rng = np.random.default_rng(seed)
+
+    def shuffle(group):
+        out = {}
+        for k in sorted(group):
+            t = group[k]
+            if t.is_floating_point():
+                t = t.reshape(-1)[torch.from_numpy(rng.permutation(t.numel()))].reshape(t.shape)
+            out[k] = t
+        return out
+    return shuffle(inputs), shuffle(params)
+
+
+def synth_linear_params(shapes, seed):
+    """Parameters for a module made of Linear layers (plus XCA's temperature), keyed and shaped like ``shapes``: weights
+    uniform in +-1/sqrt(fan_in) as nn.Linear initialises them, biases N(0, 0.05^2), temperatures in [0.5, 2); fp16-rounded."""
+    g = torch.Generator().manual_seed(2000 + seed)
+    out = {}
+    for k in sorted(shapes):
+        shape = tuple(shapes[k])
+        if k.endswith("temperature"):
+            t = torch.rand(shape, generator=g) * 1.5 + 0.5
+        elif len(shape) >= 2:
+            t = (torch.rand(shape, generator=g) * 2 - 1) / math.sqrt(math.prod(shape[1:]))
+        else:
+            t = torch.randn(shape, generator=g) * 0.05
+        out[k] = round_fp16_(t)
+    return out
+
+
+def sample_index(numel):
+    """Flat indices of the elements of a recorded output that are stored: SAMPLE of them spread evenly over the tensor (all of
+    them if it is smaller).  Plain integer arithmetic, so the same on every machine."""
+    n = min(numel, SAMPLE)
+    return np.arange(n, dtype=np.int64) * numel // n
 
 
 def p2t_d_convs(inputs, device="cpu"):

@@ -4,10 +4,13 @@ tests/golden/models/vit_tiny.npz holds the parameters, an input batch and the lo
 `ViT.VisionTransformer` (oracle/make_golden_model.py).  The model glue around the attention modules is restated in
 oracle/model_glue.py, so the same model can be evaluated where /root/reference is absent:
   * CPU: glue + oracle attention reproduces the reference logits (pins the glue);
-  * CPU, reference mounted: the drop-in class substituted into the reference's own model constructs and loads the
-    reference state_dict strictly (constructor signature + keys), and refuses to run on CPU;
+  * CPU: the drop-in class, built with the constructor arguments the reference's own model passes to the class it
+    replaces (recorded in tests/golden/reference/reference_contract.json by oracle/record_reference.py), loads the reference
+    state_dict strictly (constructor signature + keys), and refuses to run on CPU;
   * GPU: glue + B200 drop-in attention (fp16 I/O) against the reference logits.
 """
+import importlib
+import json
 import os
 import sys
 
@@ -22,7 +25,38 @@ from oracle import vit_attention  # noqa: E402
 from oracle.model_glue import attention_state, vit_model_forward  # noqa: E402
 
 CFG = dict(image_size=64, patch_size=16, in_channels=3, depths=2, num_heads=2, embedding_dim=128, num_classes=10)
-REF = "/root/reference/vision_transformers"
+with open(os.path.join(GOLDEN_DIR, "reference", "reference_contract.json")) as _f:
+    MODELS = json.load(_f)["models"]
+
+
+def _decode(v):
+    """Constructor arguments as recorded (oracle/record_reference.py:_encode): classes and partials by qualified name."""
+    if isinstance(v, list):
+        return [_decode(a) for a in v]
+    if isinstance(v, dict) and "class" in v:
+        mod, _, name = v["class"].rpartition(".")
+        return getattr(importlib.import_module(mod), name)
+    if isinstance(v, dict) and "partial" in v:
+        import functools
+        return functools.partial(_decode(v["partial"]), **{k: _decode(a) for k, a in v["kwargs"].items()})
+    return v
+
+
+def _swap_in(record, swaps):
+    """Build the drop-in for every recorded outermost constructor call the reference model made to a class in `swaps`, with
+    the same arguments.  Checks that it replaces as many reference modules as the call built and that its state_dict has the
+    reference sub-module's keys and shapes; returns [(path, drop-in)]."""
+    built = []
+    for call in record["calls"]:
+        m = swaps[call["cls"]](*_decode(call["args"]), **{k: _decode(v) for k, v in call["kwargs"].items()})
+        assert sum(isinstance(x, tuple(swaps.values())) for x in m.modules()) == call["replaced"] > 0
+        assert {k: list(v.shape) for k, v in m.state_dict().items()} == {k: s for k, (s, _) in call["state_dict"].items()}
+        built.append((call["path"], m))
+    return built
+
+
+def _sub_state(sd, path):
+    return {k[len(path) + 1:]: v for k, v in sd.items() if k.startswith(path + ".")}
 
 
 def _load():
@@ -42,25 +76,23 @@ def test_glue_with_oracle_attention_reproduces_reference_model_logits():
     assert (y - y_ref).abs().max().item() <= 2e-5 * y_ref.abs().max().item()
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference not mounted")
 @pytest.mark.parametrize("level", ["attention", "block"])
-def test_class_swap_inside_the_reference_model_constructs_and_loads(monkeypatch, level):
+def test_class_swap_inside_the_reference_model_constructs_and_loads(level):
     import pytorch_attention_b200 as pa
-    monkeypatch.syspath_prepend(REF)
-    import ViT
     if level == "attention":
-        monkeypatch.setattr(ViT, "Attention", pa.vit.Attention)    # the substitution INTEGRATION.md describes
+        swaps = {"Attention": pa.vit.Attention}                    # the substitution INTEGRATION.md describes
     else:
-        monkeypatch.setattr(ViT, "TransformerEncoder", pa.vit.TransformerEncoder)   # whole block: LN + attention + residual fused
-    model = ViT.VisionTransformer(**CFG).eval()                    # ViT.py:98 constructs the drop-in with the reference's arguments
-    assert all(isinstance(b.attn, pa.vit.Attention) for b in model.blocks)
-    if level == "block":
-        assert all(isinstance(b, pa.vit.TransformerEncoder) for b in model.blocks)
+        swaps = {"TransformerEncoder": pa.vit.TransformerEncoder}  # whole block: LN + attention + residual fused
+    # ViT.py:98 constructs the drop-in with the reference's arguments
+    built = _swap_in(MODELS["ViT.VisionTransformer(tiny):" + next(iter(swaps))], swaps)
+    assert [p for p, _ in built] == [f"blocks.{i}" + (".attn" if level == "attention" else "") for i in range(CFG["depths"])]
     sd, x, _ = _load()
-    model.load_state_dict(sd, strict=True)                         # identical keys and shapes
-    with pytest.raises(RuntimeError, match="CPU"):                 # product path: no CPU fallback
-        with torch.no_grad():
-            model(x)
+    for path, m in built:
+        assert isinstance(m if level == "attention" else m.attn, pa.vit.Attention)
+        m.eval().load_state_dict(_sub_state(sd, path), strict=True)   # identical keys and shapes
+        with pytest.raises(RuntimeError, match="CPU"):             # product path: no CPU fallback
+            with torch.no_grad():
+                m(torch.randn(2, 17, CFG["embedding_dim"]).half())
 
 
 @pytest.mark.gpu
@@ -95,25 +127,15 @@ def _swap_targets():
     }
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference not mounted")
 @pytest.mark.parametrize("modname", ["pvt", "cvt", "cswin", "xcit", "moat"])
-def test_class_swap_in_the_reference_zoo_models(modname, monkeypatch):
-    """The reference's own model constructors build the drop-ins with the reference's arguments, and a stock model's
-    state_dict loads strictly into the swapped model (same keys, same shapes) -- for every model family on the path."""
-    import importlib
-    monkeypatch.syspath_prepend(REF)
-    mod = importlib.import_module(modname)
+def test_class_swap_in_the_reference_zoo_models(modname):
+    """The drop-ins accept the arguments the reference's own model constructors pass, replace as many modules as the stock
+    model has, and hold the same state_dict keys and shapes -- for every model family on the path."""
     factory, swaps = _swap_targets()[modname]
-    torch.manual_seed(0)
-    stock = getattr(mod, factory)()
-    sd = stock.state_dict()
-    for name, cls in swaps.items():
-        monkeypatch.setattr(mod, name, cls)
-    swapped = getattr(mod, factory)()
-    n_dropins = sum(isinstance(m, tuple(swaps.values())) for m in swapped.modules())
-    n_stock = sum(type(m).__name__ in swaps for m in stock.modules())
-    assert n_dropins == n_stock and n_dropins > 0
-    swapped.load_state_dict(sd, strict=True)
+    record = MODELS[f"{modname}.{factory}()"]
+    assert {c["cls"] for c in record["calls"]} <= set(swaps)
+    for call, (_, m) in zip(record["calls"], _swap_in(record, swaps)):
+        m.load_state_dict({k: torch.zeros(s, dtype=getattr(torch, dt)) for k, (s, dt) in call["state_dict"].items()}, strict=True)
 
 
 # ---------------------------------------------------------------- the reference's DEFAULT model: VisionTransformer()
@@ -139,16 +161,17 @@ def test_default_model_glue_with_oracle_attention_reproduces_reference_logits():
     assert (y - y_ref).abs().max().item() <= 5e-5 * y_ref.abs().max().item()
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference not mounted")
-def test_default_reference_model_accepts_the_dropin_and_the_synthetic_state(monkeypatch):
+def test_default_reference_model_accepts_the_dropin_and_the_synthetic_state():
     import pytorch_attention_b200 as pa
     from oracle.model_glue import vit_state_shapes, synth_state_dict
-    monkeypatch.syspath_prepend(REF)
-    import ViT
-    monkeypatch.setattr(ViT, "Attention", pa.vit.Attention)
-    model = ViT.VisionTransformer()                                # every default: 4 heads of 192
-    assert all(b.attn.num_heads == 4 for b in model.blocks)
-    model.load_state_dict(synth_state_dict(vit_state_shapes(), 77), strict=True)
+    record = MODELS["ViT.VisionTransformer():Attention"]           # every default: 4 heads of 192
+    shapes = vit_state_shapes()
+    assert {k: list(s) for k, s in shapes.items()} == {k: s for k, (s, _) in record["state_dict"].items()}
+    built = _swap_in(record, {"Attention": pa.vit.Attention})
+    assert len(built) == 12 and all(m.num_heads == 4 for _, m in built)
+    sd = synth_state_dict(shapes, 77)
+    for path, m in built:
+        m.load_state_dict(_sub_state(sd, path), strict=True)
 
 
 @pytest.mark.gpu

@@ -1,22 +1,39 @@
 """Host-side contract of the drop-in modules (no GPU): constructor signatures, state_dict keys/shapes,
 error behaviour, and no silent CPU fallback."""
 import inspect
+import json
 import os
-import sys
 
 import pytest
 import torch
 
 import pytorch_attention_b200 as pa
+from _util import GOLDEN_DIR
 
-REF = os.environ.get("PA_REFERENCE", "/root/reference/vision_transformers")
-HAVE_REF = os.path.isdir(REF)
+# signatures and state_dict shapes of the reference classes, recorded by oracle/record_reference.py
+with open(os.path.join(GOLDEN_DIR, "reference", "reference_contract.json")) as _f:
+    CONTRACT = json.load(_f)["classes"]
 
 
-def _ref(mod):
-    if REF not in sys.path:
-        sys.path.insert(0, REF)
-    return __import__(mod)
+class _Ref:
+    """What was recorded of one reference class: its signatures and, per constructor call, its state_dict and attributes."""
+
+    def __init__(self, name):
+        self.name, self.entry = name, CONTRACT[name]
+        self.init, self.forward = self.entry["init"], self.entry["forward"]
+
+    def __call__(self, **kw):
+        key = f"{self.name}(" + ", ".join(f"{k}={v!r}" for k, v in kw.items()) + ")"
+        return self.entry["instances"][key]
+
+
+def _ref_state_dict(inst):
+    """Zero tensors with the recorded keys, shapes and dtypes of a reference module's state_dict."""
+    return {k: torch.zeros(shape, dtype=getattr(torch, dt)) for k, (shape, dt) in inst["state_dict"].items()}
+
+
+def _shapes(inst):
+    return {k: torch.Size(shape) for k, (shape, _) in inst["state_dict"].items()}
 
 
 def test_vit_state_dict_keys_and_shapes():
@@ -57,14 +74,13 @@ def test_unsupported_modes_raise():
         check_forward_mode(m.eval(), Fake(), (0.1,))
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="reference not mounted")
 def test_vit_matches_live_reference_contract():
-    ref = _ref("ViT").Attention
-    assert str(inspect.signature(ref.__init__)) == str(inspect.signature(pa.ViTAttention.__init__))
-    r = ref(192, 3, qkv_bias=True)
+    ref = _Ref("ViT.Attention")
+    assert ref.init == str(inspect.signature(pa.ViTAttention.__init__))
+    r = ref(dim=192, num_heads=3, qkv_bias=True)
     m = pa.ViTAttention(192, 3, qkv_bias=True)
-    assert {k: v.shape for k, v in r.state_dict().items()} == {k: v.shape for k, v in m.state_dict().items()}
-    m.load_state_dict(r.state_dict())          # reference weights load unchanged
+    assert _shapes(r) == {k: v.shape for k, v in m.state_dict().items()}
+    m.load_state_dict(_ref_state_dict(r))          # reference weights load unchanged
 
 
 def test_setr_moat_defaults_and_keys():
@@ -77,17 +93,15 @@ def test_setr_moat_defaults_and_keys():
             cls(100, 3)
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="reference not mounted")
 @pytest.mark.parametrize("modname", ["setr", "moat"])
 def test_setr_moat_match_live_reference_contract(modname):
-    from oracle.cases import load_reference_class
-    ref = load_reference_class(REF, modname, "Attention")
+    ref = _Ref(f"{modname}.Attention")
     ours = getattr(pa, modname).Attention
-    assert str(inspect.signature(ref.__init__)) == str(inspect.signature(ours.__init__))
-    r = ref(256, qkv_bias=True)
+    assert ref.init == str(inspect.signature(ours.__init__))
+    r = ref(dim=256, qkv_bias=True)
     m = ours(256, qkv_bias=True)
-    assert {k: v.shape for k, v in r.state_dict().items()} == {k: v.shape for k, v in m.state_dict().items()}
-    m.load_state_dict(r.state_dict())
+    assert _shapes(r) == {k: v.shape for k, v in m.state_dict().items()}
+    m.load_state_dict(_ref_state_dict(r))
 
 
 def test_param_stage_is_dropped_when_parameters_may_have_changed():
@@ -150,84 +164,75 @@ def test_segformer_cmt_keys_and_defaults():
         pa.cmt.Attention(100, 3)
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="reference not mounted")
 @pytest.mark.parametrize("modname,cls,kw", [
     ("segformer", "Attention", dict(dim=64, num_heads=2, qkv_bias=True, sr_ratio=4)),
     ("cmt", "Attention", dict(dim=128, num_heads=2, sr_ratio=2, qkv_bias=True)),
     ("pvt", "Block", dict(dim=128, num_heads=2, sr_ratio=4)),
 ])
 def test_siblings_match_live_reference_contract(modname, cls, kw):
-    ref = getattr(_ref(modname), cls)
+    ref = _Ref(f"{modname}.{cls}")
     ours = getattr(getattr(pa, modname), cls)
-    assert str(inspect.signature(ref.__init__)) == str(inspect.signature(ours.__init__))
+    assert ref.init == str(inspect.signature(ours.__init__))
     if cls == "Attention":
-        assert str(inspect.signature(ref.forward)) == str(inspect.signature(ours.forward))
+        assert ref.forward == str(inspect.signature(ours.forward))
     r, m = ref(**kw), ours(**kw)
-    assert {k: v.shape for k, v in r.state_dict().items()} == {k: v.shape for k, v in m.state_dict().items()}
-    m.load_state_dict(r.state_dict())          # reference weights load unchanged
+    assert _shapes(r) == {k: v.shape for k, v in m.state_dict().items()}
+    m.load_state_dict(_ref_state_dict(r))          # reference weights load unchanged
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="reference not mounted")
 def test_xca_block_attention_half_loads_a_reference_block():
     """XCABlockAttentionHalf holds the attention half's parameters under XCABlock's own keys (xcit.py:267-291)."""
-    blk = _ref("xcit").XCABlock(128, 4, qkv_bias=True, eta=1.0)
+    blk = _Ref("xcit.XCABlock")(dim=128, num_heads=4, qkv_bias=True, eta=1.0)
     m = pa.xcit.XCABlockAttentionHalf(128, 4, qkv_bias=True, eta=1.0)
-    res = m.load_state_dict(blk.state_dict(), strict=False)
+    res = m.load_state_dict(_ref_state_dict(blk), strict=False)
     assert not res.missing_keys
     assert all(k.split(".")[0] in ("norm2", "norm3", "mlp", "local_mp", "gamma2", "gamma3") for k in res.unexpected_keys)
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="reference not mounted")
 @pytest.mark.parametrize("kw", [dict(dim=192, heads=3, dim_head=64), dict(dim=64, heads=1, dim_head=64)])
 def test_bvit_broad_attention_matches_live_reference_contract(kw):
-    ref = _ref("bvit").Broad_Attention
-    assert str(inspect.signature(ref.__init__)) == str(inspect.signature(pa.bvit.Broad_Attention.__init__))
+    ref = _Ref("bvit.Broad_Attention")
+    assert ref.init == str(inspect.signature(pa.bvit.Broad_Attention.__init__))
     r, m = ref(**kw), pa.bvit.Broad_Attention(**kw)
-    assert {k: v.shape for k, v in r.state_dict().items()} == {k: v.shape for k, v in m.state_dict().items()}
-    m.load_state_dict(r.state_dict())
-    assert isinstance(m.to_out, torch.nn.Identity) == isinstance(r.to_out, torch.nn.Identity)
+    assert _shapes(r) == {k: v.shape for k, v in m.state_dict().items()}
+    m.load_state_dict(_ref_state_dict(r))
+    assert isinstance(m.to_out, torch.nn.Identity) == r["to_out_is_identity"]
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="reference not mounted")
 def test_pam_matches_live_reference_contract():
-    from oracle.cases import load_reference_class
-    ref = load_reference_class(REF, "dual_attention", "PAM")
-    assert str(inspect.signature(ref.__init__)) == str(inspect.signature(pa.dual_attention.PAM.__init__))
-    r, m = ref(64), pa.dual_attention.PAM(64)
-    assert {k: v.shape for k, v in r.state_dict().items()} == {k: v.shape for k, v in m.state_dict().items()}
-    m.load_state_dict(r.state_dict())
+    ref = _Ref("dual_attention.PAM")
+    assert ref.init == str(inspect.signature(pa.dual_attention.PAM.__init__))
+    r, m = ref(dim=64), pa.dual_attention.PAM(64)
+    assert _shapes(r) == {k: v.shape for k, v in m.state_dict().items()}
+    m.load_state_dict(_ref_state_dict(r))
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="reference not mounted")
 def test_dilateformer_global_attention_matches_live_reference_contract():
-    from oracle.cases import load_reference_class
-    ref = load_reference_class(REF, "dilateformer", "GlobalAttention")
+    ref = _Ref("dilateformer.GlobalAttention")
     ours = pa.dilateformer.GlobalAttention
-    assert str(inspect.signature(ref.__init__)) == str(inspect.signature(ours.__init__))
-    r, m = ref(128, 2, qkv_bias=True), ours(128, 2, qkv_bias=True)
-    assert {k: v.shape for k, v in r.state_dict().items()} == {k: v.shape for k, v in m.state_dict().items()}
-    m.load_state_dict(r.state_dict())
-    assert ours(128, 2, qk_scale=0.25).scale == ref(128, 2, qk_scale=0.25).scale == 0.25
+    assert ref.init == str(inspect.signature(ours.__init__))
+    r, m = ref(dim=128, num_heads=2, qkv_bias=True), ours(128, 2, qkv_bias=True)
+    assert _shapes(r) == {k: v.shape for k, v in m.state_dict().items()}
+    m.load_state_dict(_ref_state_dict(r))
+    assert ours(128, 2, qk_scale=0.25).scale == ref.entry["qk_scale_0.25"] == 0.25
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="reference not mounted")
 def test_p2t_pooling_attention_matches_live_reference_contract():
-    ref = _ref("p2t").PoolingAttention
+    ref = _Ref("p2t.PoolingAttention")
     ours = pa.p2t.PoolingAttention
-    assert str(inspect.signature(ref.__init__)) == str(inspect.signature(ours.__init__))
-    assert str(inspect.signature(ref.forward)) == str(inspect.signature(ours.forward))
-    r, m = ref(128, 2, qkv_bias=True), ours(128, 2, qkv_bias=True)
-    assert {k: v.shape for k, v in r.state_dict().items()} == {k: v.shape for k, v in m.state_dict().items()}
-    m.load_state_dict(r.state_dict())
-    assert m.num_elements == r.num_elements
+    assert ref.init == str(inspect.signature(ours.__init__))
+    assert ref.forward == str(inspect.signature(ours.forward))
+    r, m = ref(dim=128, num_heads=2, qkv_bias=True), ours(128, 2, qkv_bias=True)
+    assert _shapes(r) == {k: v.shape for k, v in m.state_dict().items()}
+    m.load_state_dict(_ref_state_dict(r))
+    assert m.num_elements == r["num_elements"]
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="reference not mounted")
 def test_kvt_knn_attention_matches_live_reference_contract():
-    ref = _ref("kvt").KNNAttention
+    ref = _Ref("kvt.KNNAttention")
     ours = pa.kvt.KNNAttention
-    assert str(inspect.signature(ref.__init__)) == str(inspect.signature(ours.__init__))
-    r, m = ref(128, 2, qkv_bias=True, topk=50), ours(128, 2, qkv_bias=True, topk=50)
-    assert {k: v.shape for k, v in r.state_dict().items()} == {k: v.shape for k, v in m.state_dict().items()}
-    m.load_state_dict(r.state_dict())
-    assert m.topk == r.topk == 50
+    assert ref.init == str(inspect.signature(ours.__init__))
+    r, m = ref(dim=128, num_heads=2, qkv_bias=True, topk=50), ours(128, 2, qkv_bias=True, topk=50)
+    assert _shapes(r) == {k: v.shape for k, v in m.state_dict().items()}
+    m.load_state_dict(_ref_state_dict(r))
+    assert m.topk == r["topk"] == 50

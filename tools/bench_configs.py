@@ -15,7 +15,6 @@ import pytorch_attention_b200 as pa  # noqa: E402
 from pytorch_attention_b200 import _lib  # noqa: E402
 
 OUT = os.path.join(ROOT, "gpurun_out")
-os.makedirs(OUT, exist_ok=True)
 PEAK = 1704.0
 try:
     PEAK = json.load(open(os.path.join(ROOT, "MEASURED_PEAKS.json")))["bf16_tflops"]
@@ -50,6 +49,7 @@ def emit(**kw):
         return
     line = json.dumps(kw)
     print(line, flush=True)
+    os.makedirs(OUT, exist_ok=True)
     with open(os.path.join(OUT, "configs.jsonl"), "a") as f:
         f.write(line + "\n")
 
