@@ -7,6 +7,8 @@
  *     cvt.Attention.forward            cvt.py:64-76      -> pa_cvt_fwd
  *     cswin.LePEAttention.forward      cswin.py:101-127  -> pa_cswin_lepe_fwd
  *     cswin.CSWinBlock.forward (attn)  cswin.py:176-194  -> pa_cswin_block_attn_fwd
+ *     dilateformer.MultiDilatelocalAttention.forward  dilateformer.py:85-97 -> pa_dilate_fwd
+ *     dilateformer.DilateBlock.forward (attn)         dilateformer.py:130   -> pa_dilate_block_attn_fwd
  *     xcit.XCA.forward                 xcit.py:245-265   -> pa_xca_fwd
  *     xcit.ClassAttention.forward      xcit.py:174-188   -> pa_class_attn_fwd
  * The reference has no FFI of its own (it is pure Python calling ATen); these entry points are what a
@@ -312,6 +314,52 @@ typedef struct {
 } pa_cswin_block_args;
 size_t pa_cswin_block_attn_workspace_bytes(const pa_cswin_block_args* a);
 int pa_cswin_block_attn_fwd(const pa_cswin_block_args* a, void* workspace, size_t workspace_bytes, void* stream);
+
+/* ---------------------------------------------------------------- dilateformer.MultiDilatelocalAttention (dilateformer.py:41-97) */
+/* Multi-scale dilated attention on a channels-last image x[B, Himg, Wimg, C].  qkv = 1x1 conv (a token-major GEMM), column
+ * s*C + g*Cg + h*hd + d = (q/k/v, dilation group g, head h of the group, channel d), Cg = C / n_dilation.  Query (y, x) of group g
+ * attends to the kernel_size^2 keys at (y + i*dilation[g] - p, x + j*dilation[g] - p), p = dilation[g]*(kernel_size-1)/2
+ * (nn.Unfold, zero padding: a key outside the map has logit 0 and value 0 and still takes part in the softmax); the result of
+ * head h of group g lands at column g*Cg + h*hd + d, and y = proj(O) + proj_bias.  head_dim = C / H a multiple of 8 up to 64,
+ * odd kernel_size <= 7 (an even one is PA_ERR_BAD_SHAPE), 1 to 8 groups, H % n_dilation == 0, any dilation >= 1 (one beyond the
+ * map is all padding but the centre tap).  Width bound: a CTA stages whole image rows of its group, so for every group
+ * 4 * Wimg * pitch * min(Himg, 1 + dilation*(kernel_size-1), kernel_size) bytes must fit 227 KB, pitch = Cg rounded up to an
+ * odd multiple of 8; at kernel_size 3 that is Wimg <= 807 for Cg 24, 484 for Cg 32, 345 for Cg 48.  Wider maps:
+ * PA_ERR_UNSUPPORTED.
+ * Launches: GEMM(qkv) -> dilated-attention kernel -> GEMM(proj).
+ * The reference writes the pre-projection attention output into the caller's x (dilateformer.py:90-93 assign through a view of a
+ * contiguous x); this library reads x only. */
+typedef struct {
+  int dtype, out_dtype;      /* x and qkv_weight: F16/BF16; y: F16/BF16/F32 */
+  int B, Himg, Wimg, C, H;   /* H = num_heads */
+  int kernel_size, n_dilation;
+  int dilation[8];           /* dilation[g], g < n_dilation */
+  float scale;               /* qk_scale or head_dim ** -0.5 (dilateformer.py:75) */
+  const void* x;             /* [B,Himg,Wimg,C] */
+  const void* qkv_weight;    /* [3C,C] (dtype): qkv.weight [3C,C,1,1] */
+  const float* qkv_bias;     /* [3C] or NULL */
+  const void* proj_weight;   /* [C,C] fp16 */
+  const float* proj_bias;    /* [C] or NULL */
+  void* y;                   /* [B,Himg,Wimg,C] */
+} pa_dilate_args;
+size_t pa_dilate_workspace_bytes(const pa_dilate_args* a);
+int pa_dilate_fwd(const pa_dilate_args* a, void* workspace, size_t workspace_bytes, void* stream);
+/* The dilated-attention kernel alone: o[B*Himg*Wimg, C] from a caller's qkv[B*Himg*Wimg, 3C] (both fp16, 16-byte aligned, laid out
+ * as above).  Uses B, Himg, Wimg, C, H, kernel_size, n_dilation, dilation and scale of `a`. */
+int pa_dilate_core(const pa_dilate_args* a, const void* qkv, void* o, void* stream);
+
+/* ---------------------------------------------------------------- dilateformer.DilateBlock, attention half (dilateformer.py:126-130) */
+/* y = x + MultiDilatelocalAttention(LayerNorm(x)) on channels-last x: this library's LayerNorm row kernel (fp32 statistics, fp16
+ * output) in front, the residual x added in the epilogue of the proj GEMM.  attn.qkv_weight must be fp16 (its input is the fp16
+ * LayerNorm output).  Launches: LayerNorm -> GEMM(qkv) -> dilated-attention kernel -> GEMM(proj + residual). */
+typedef struct {
+  pa_dilate_args attn;       /* attn.x = block input (channels-last), attn.y = block output of the attention half */
+  const float* ln_weight;    /* [C] norm1.weight */
+  const float* ln_bias;      /* [C] norm1.bias */
+  float ln_eps;
+} pa_dilate_block_args;
+size_t pa_dilate_block_attn_workspace_bytes(const pa_dilate_block_args* a);
+int pa_dilate_block_attn_fwd(const pa_dilate_block_args* a, void* workspace, size_t workspace_bytes, void* stream);
 
 #ifdef __cplusplus
 }

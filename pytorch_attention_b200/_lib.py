@@ -101,6 +101,16 @@ class CswinBlockArgs(C.Structure):
                 ("y", _vp)]
 
 
+class DilateArgs(C.Structure):
+    _fields_ = [("dtype", _i), ("out_dtype", _i), ("B", _i), ("Himg", _i), ("Wimg", _i), ("C", _i), ("H", _i),
+                ("kernel_size", _i), ("n_dilation", _i), ("dilation", _i * 8), ("scale", _f),
+                ("x", _vp), ("qkv_weight", _vp), ("qkv_bias", _vp), ("proj_weight", _vp), ("proj_bias", _vp), ("y", _vp)]
+
+
+class DilateBlockArgs(C.Structure):
+    _fields_ = [("attn", DilateArgs), ("ln_weight", _vp), ("ln_bias", _vp), ("ln_eps", _f)]
+
+
 # name -> (restype, argtypes); every symbol declared in include/pa_b200.h must be listed here
 # (tests/test_abi.py cross-checks this table against the header).
 SYMBOLS = {
@@ -138,6 +148,11 @@ SYMBOLS = {
     "pa_cswin_lepe_fwd": (_i, [C.POINTER(LepeArgs), _vp]),
     "pa_cswin_block_attn_workspace_bytes": (C.c_size_t, [C.POINTER(CswinBlockArgs)]),
     "pa_cswin_block_attn_fwd": (_i, [C.POINTER(CswinBlockArgs), _vp, C.c_size_t, _vp]),
+    "pa_dilate_workspace_bytes": (C.c_size_t, [C.POINTER(DilateArgs)]),
+    "pa_dilate_fwd": (_i, [C.POINTER(DilateArgs), _vp, C.c_size_t, _vp]),
+    "pa_dilate_core": (_i, [C.POINTER(DilateArgs), _vp, _vp, _vp]),
+    "pa_dilate_block_attn_workspace_bytes": (C.c_size_t, [C.POINTER(DilateBlockArgs)]),
+    "pa_dilate_block_attn_fwd": (_i, [C.POINTER(DilateBlockArgs), _vp, C.c_size_t, _vp]),
 }
 
 _lock = threading.Lock()

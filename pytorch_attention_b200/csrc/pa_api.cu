@@ -9,6 +9,7 @@
 #include "pa_xca.cuh"
 #include "pa_attn_win.cuh"
 #include "pa_attn_proj.cuh"
+#include "pa_dilate.cuh"
 
 #include <math.h>
 #include <stdlib.h>
@@ -1733,6 +1734,174 @@ int pa_cswin_block_attn_fwd(const pa_cswin_block_args* a, void* workspace, size_
   // y = x + proj(att)   (cswin.py:193-194)
   return linear(att, PA_DTYPE_F16, C, a->proj_weight, PA_DTYPE_F16, a->proj_bias, a->y, a->out_dtype, C, rows, C, C, st,
                 a->residual ? a->x : nullptr, C, a->dtype);
+}
+
+// ================================================================ DilateFormer multi-scale dilated attention  (dilateformer.py:41-134)
+static int dilate_check(const pa_dilate_args* a, const char* who) {
+  if (!a) return fail(PA_ERR_NULL, "%s: args is NULL", who);
+  if (a->B <= 0 || a->Himg <= 0 || a->Wimg <= 0 || a->C <= 0 || a->H <= 0) return fail(PA_ERR_BAD_SHAPE, "%s: B,H,W,C,num_heads must be positive", who);
+  if (a->B > 65535) return fail(PA_ERR_UNSUPPORTED, "%s: batch %d exceeds 65535 images per call", who, a->B);
+  if (a->n_dilation < 1 || a->n_dilation > DL_MAX_GROUPS)
+    return fail(PA_ERR_UNSUPPORTED, "%s: %d dilation groups (1 to %d supported)", who, a->n_dilation, DL_MAX_GROUPS);
+  if (a->H % a->n_dilation)
+    return fail(PA_ERR_BAD_SHAPE, "%s: num_heads%d must be the times of num_dilation%d (dilateformer.py:77)", who, a->H, a->n_dilation);
+  if (a->C % a->H) return fail(PA_ERR_BAD_SHAPE, "%s: dim %d not divisible by num_heads %d", who, a->C, a->H);
+  if (a->kernel_size < 1 || a->kernel_size % 2 == 0)
+    return fail(PA_ERR_BAD_SHAPE, "%s: kernel_size %d must be odd (an even kernel's unfold output does not reshape, dilateformer.py:55)", who, a->kernel_size);
+  if (a->kernel_size > 7) return fail(PA_ERR_UNSUPPORTED, "%s: kernel_size %d unsupported (odd, up to 7)", who, a->kernel_size);
+  for (int g = 0; g < a->n_dilation; ++g)
+    if (a->dilation[g] < 1) return fail(PA_ERR_BAD_SHAPE, "%s: dilation[%d] = %d must be >= 1", who, g, a->dilation[g]);
+  const int hd = a->C / a->H;
+  if (hd % 8 || hd > 64) return fail(PA_ERR_UNSUPPORTED, "%s: head_dim %d unsupported (multiples of 8 up to 64)", who, hd);
+  if (!(a->scale > 0.f)) return fail(PA_ERR_UNSUPPORTED, "%s: scale must be > 0", who);
+  if (a->dtype != PA_DTYPE_F16 && a->dtype != PA_DTYPE_BF16) return fail(PA_ERR_UNSUPPORTED, "%s: dtype must be fp16/bf16", who);
+  if (a->out_dtype < PA_DTYPE_F16 || a->out_dtype > PA_DTYPE_F32) return fail(PA_ERR_UNSUPPORTED, "%s: bad out_dtype", who);
+  return PA_OK;
+}
+
+// Band height and shared memory of the dilated-attention kernel: 8 image rows per CTA, halved until the widest group's staged
+// rows (at most kernel_size * band rows, whatever the dilation) fit 113 KB; when a single band row does not fit 227 KB the map
+// is too wide for this group width: 4 * Wimg * pitch * min(Himg, 1 + dil*(k-1), k) bytes must fit (pa_b200.h).
+static int dilate_plan(const pa_dilate_args* a, DilateParams* p, int* smem) {
+  const int Cg = a->C / a->n_dilation;
+  p->Cg = Cg;
+  p->heads_g = a->H / a->n_dilation;
+  p->pstride = (Cg / 8) % 2 ? Cg : Cg + 8;
+  const int dmax = a->Himg > a->Wimg ? a->Himg : a->Wimg;
+  for (int g = 0; g < a->n_dilation; ++g)   // a dilation >= max(H, W) puts every tap but the centre outside the map: same result
+    p->dil[g] = a->dilation[g] < dmax ? a->dilation[g] : dmax;
+  auto rows_for = [&](int rows) {
+    int r = 0;
+    for (int g = 0; g < a->n_dilation; ++g) {
+      const int rg = dilate_staged_rows(rows, a->kernel_size, p->dil[g], a->Himg);
+      r = rg > r ? rg : r;
+    }
+    return r;
+  };
+  auto bytes = [&](int rows) { return 2ll * rows_for(rows) * a->Wimg * p->pstride * 2; };
+  int rows = a->Himg < 8 ? a->Himg : 8;
+  while (rows > 1 && bytes(rows) > 113 * 1024) rows /= 2;
+  if (bytes(rows) > 227 * 1024)
+    return fail(PA_ERR_UNSUPPORTED, "pa_dilate: %d staged rows of %d pixels x %d channels exceed shared memory (map too wide)",
+                rows_for(rows), a->Wimg, Cg);
+  p->rows = rows;
+  *smem = (int)bytes(rows);
+  return PA_OK;
+}
+
+extern "C++" template <int HD>
+int launch_dilate_t(const DilateParams& p, int smem, int ng, cudaStream_t st) {
+  static SmemAttr attr;
+  int rc = attr.ensure(dilate_attn_kernel<HD>, smem);
+  if (rc) return rc;
+  dim3 grid((p.Himg + p.rows - 1) / p.rows, ng, p.B);
+  dilate_attn_kernel<HD><<<grid, DL_THREADS, smem, st>>>(p);
+  PA_CUDA_OK(cudaGetLastError());
+  launch_counter()++;
+  return PA_OK;
+}
+
+// O[B*H*W, C] = dilated attention of qkv[B*H*W, 3C] (both fp16, 16-byte aligned); arguments already checked by dilate_check.
+// Plans (shared memory) and checks the device before the launch.
+static int dilate_launch(const pa_dilate_args* a, const void* qkv, void* o, cudaStream_t st) {
+  if ((reinterpret_cast<uintptr_t>(qkv) & 15) || (reinterpret_cast<uintptr_t>(o) & 15))
+    return fail(PA_ERR_MISALIGNED, "pa_dilate: qkv / O buffers must be 16-byte aligned");
+  DilateParams p = {};
+  int smem = 0, rc;
+  if ((rc = dilate_plan(a, &p, &smem))) return rc;
+  if ((rc = current_device_check())) return rc;
+  p.qkv = reinterpret_cast<const uint16_t*>(qkv);
+  p.o = reinterpret_cast<uint16_t*>(o);
+  p.B = a->B; p.Himg = a->Himg; p.Wimg = a->Wimg; p.C = a->C; p.ks = a->kernel_size;
+  p.scale_log2 = a->scale * 1.4426950408889634f;
+  switch (a->C / a->H) {
+    case 8:  return launch_dilate_t<8>(p, smem, a->n_dilation, st);
+    case 16: return launch_dilate_t<16>(p, smem, a->n_dilation, st);
+    case 24: return launch_dilate_t<24>(p, smem, a->n_dilation, st);
+    case 32: return launch_dilate_t<32>(p, smem, a->n_dilation, st);
+    case 40: return launch_dilate_t<40>(p, smem, a->n_dilation, st);
+    case 48: return launch_dilate_t<48>(p, smem, a->n_dilation, st);
+    case 56: return launch_dilate_t<56>(p, smem, a->n_dilation, st);
+    case 64: return launch_dilate_t<64>(p, smem, a->n_dilation, st);
+    default: return fail(PA_ERR_UNSUPPORTED, "pa_dilate: head_dim %d unsupported", a->C / a->H);
+  }
+}
+
+int pa_dilate_core(const pa_dilate_args* a, const void* qkv, void* o, void* stream) {
+  int rc = dilate_check(a, "pa_dilate_core");
+  if (rc) return rc;
+  if (!qkv || !o) return fail(PA_ERR_NULL, "pa_dilate_core: qkv/o must be non-NULL");
+  return dilate_launch(a, qkv, o, (cudaStream_t)stream);
+}
+
+size_t pa_dilate_workspace_bytes(const pa_dilate_args* a) {
+  if (dilate_check(a, "pa_dilate")) return 0;
+  const size_t rows = (size_t)a->B * a->Himg * a->Wimg;
+  return align_up(rows * 3 * a->C * 2, 1024) + align_up(rows * a->C * 2, 1024) + 1024;
+}
+
+// qkv GEMM -> dilated attention -> proj GEMM (+ residual in its epilogue).  x_in: the qkv GEMM's A operand (a->x, or the
+// LayerNorm output of the block entry point); residual: nullptr or the block input (dtype a->dtype, pitch C).
+static int dilate_run(const pa_dilate_args* a, const void* x_in, int x_dtype, const void* residual, Arena& ws, cudaStream_t st) {
+  int rc;
+  const int C = a->C;
+  const long long rows = (long long)a->B * a->Himg * a->Wimg;
+  void* qkv = ws.take((size_t)rows * 3 * C * 2);
+  void* obuf = ws.take((size_t)rows * C * 2);
+  // qkv = 1x1 conv (dilateformer.py:88) on channels-last tokens: a token-major GEMM with the [3C, C] weight
+  if ((rc = linear(x_in, x_dtype, C, a->qkv_weight, x_dtype, a->qkv_bias, qkv, PA_DTYPE_F16, 3 * C, rows, 3 * C, C, st))) return rc;
+  if ((rc = dilate_launch(a, qkv, obuf, st))) return rc;
+  // y = proj(O) (+ x)   (dilateformer.py:95, 130)
+  return linear(obuf, PA_DTYPE_F16, C, a->proj_weight, PA_DTYPE_F16, a->proj_bias, a->y, a->out_dtype, C, rows, C, C, st,
+                residual, C, a->dtype);
+}
+
+int pa_dilate_fwd(const pa_dilate_args* a, void* workspace, size_t workspace_bytes, void* stream) {
+  int rc = dilate_check(a, "pa_dilate_fwd");
+  if (rc) return rc;
+  if (!a->x || !a->qkv_weight || !a->proj_weight || !a->y) return fail(PA_ERR_NULL, "pa_dilate_fwd: x/qkv_weight/proj_weight/y must be non-NULL");
+  DilateParams p = {};
+  int smem = 0;
+  if ((rc = dilate_plan(a, &p, &smem))) return rc;
+  const size_t need = pa_dilate_workspace_bytes(a);
+  if (!workspace || workspace_bytes < need) return fail(PA_ERR_WORKSPACE, "pa_dilate_fwd: workspace %zu B < required %zu B", workspace_bytes, need);
+  if ((rc = current_device_check())) return rc;
+  Arena ws(workspace);
+  return dilate_run(a, a->x, a->dtype, nullptr, ws, (cudaStream_t)stream);
+}
+
+size_t pa_dilate_block_attn_workspace_bytes(const pa_dilate_block_args* b) {
+  if (!b || dilate_check(&b->attn, "pa_dilate_block")) return 0;
+  const size_t rows = (size_t)b->attn.B * b->attn.Himg * b->attn.Wimg;
+  return align_up(rows * b->attn.C * 2, 1024) + pa_dilate_workspace_bytes(&b->attn);
+}
+
+int pa_dilate_block_attn_fwd(const pa_dilate_block_args* b, void* workspace, size_t workspace_bytes, void* stream) {
+  if (!b) return fail(PA_ERR_NULL, "pa_dilate_block_attn_fwd: args is NULL");
+  const pa_dilate_args* a = &b->attn;
+  int rc = dilate_check(a, "pa_dilate_block_attn_fwd");
+  if (rc) return rc;
+  if (!a->x || !a->qkv_weight || !a->proj_weight || !a->y || !b->ln_weight || !b->ln_bias)
+    return fail(PA_ERR_NULL, "pa_dilate_block_attn_fwd: x/qkv_weight/proj_weight/y/ln_weight/ln_bias must be non-NULL");
+  DilateParams p = {};
+  int smem = 0;
+  if ((rc = dilate_plan(a, &p, &smem))) return rc;
+  const size_t need = pa_dilate_block_attn_workspace_bytes(b);
+  if (!workspace || workspace_bytes < need)
+    return fail(PA_ERR_WORKSPACE, "pa_dilate_block_attn_fwd: workspace %zu B < required %zu B", workspace_bytes, need);
+  if ((rc = current_device_check())) return rc;
+  cudaStream_t st = (cudaStream_t)stream;
+  const long long rows = (long long)a->B * a->Himg * a->Wimg;
+  Arena ws(workspace);
+  void* img = ws.take((size_t)rows * a->C * 2);
+  // img = norm1(x)   (dilateformer.py:130), fp16
+  LnParams ln;
+  ln.x = a->x; ln.out = img; ln.gamma = b->ln_weight; ln.beta = b->ln_bias; ln.rows = rows; ln.C = a->C; ln.dtype = a->dtype; ln.eps = b->ln_eps;
+  launch_layernorm(ln, st);
+  PA_CUDA_OK(cudaGetLastError());
+  launch_counter()++;
+  // x + proj(attention(img)): the residual rides in the proj GEMM's epilogue
+  return dilate_run(a, img, PA_DTYPE_F16, a->x, ws, st);
 }
 
 }  // extern "C"
